@@ -54,7 +54,18 @@ def parse_args():
     ap.add_argument("--pipeline", action="store_true",
                     help="N>1: two batches in flight (exchange of batch i under the search of batch i+1) instead of search -> exchange -> merge back to "
                          "back; measured 1.5 %% SLOWER at N=2 (profiles/r01c_bench_2M_n2_pipelined.json): the in-line exchange costs 0.02 ms of a 1.63 ms step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="--impl ours: after the timed steps, rank 0 writes what the last timed step returned (ids, scores, counts; parts when N>1) as DIR/<name>.npy "
+                         "in float64 (ids and counts) or float32 (scores), so that two builds can be compared output for output on the same inputs")
     return ap.parse_args()
+
+
+def dump_outputs(directory, names, tensors):
+    """The tensors of one search result as DIR/<name>.npy: integer arrays as float64 (exact for every int32), float32 as is."""
+    os.makedirs(directory, exist_ok=True)
+    for name, t in zip(names, tensors):
+        a = t.cpu().numpy()
+        np.save(os.path.join(directory, f"{name}.npy"), a if a.dtype == np.float32 else a.astype(np.float64))
 
 
 # ---- synthetic data (BASELINE.md §3 "synthetic embeddings of the named shape") ----------------------
@@ -473,6 +484,7 @@ def main():
         return seg.search(queries[i], k, ef=ef, method=_lib.NIDX_METHOD_HNSW, out=out)
 
     def run_steps(first, last):
+        """-> the result of the last step when pipelined."""
         if not pipelined:
             for i in range(first, last):
                 step(i)
@@ -481,7 +493,7 @@ def main():
             sharded.submit(queries[i], ef)
             if i > first:
                 sharded.collect()
-        sharded.collect()
+        return sharded.collect()
 
     # ---- warm-up + timed region: inputs resident in HBM (value) --------------------------------------
     # Everything with a host-side cost that differs between ranks (NVML initialisation: 8 processes contend for it on an
@@ -500,14 +512,16 @@ def main():
         torch.cuda.cudart().cudaProfilerStart()  # `ncu --profile-from-start off` captures exactly the timed region
         step_ev[0].record()
         if pipelined:
-            run_steps(args.warmup, n_batches)
+            last = run_steps(args.warmup, n_batches)
         else:
             for i in range(args.warmup, n_batches):
-                step(i)
+                last = step(i)
                 step_ev[i - args.warmup + 1].record()
         step_ev[-1].record()
         torch.cuda.synchronize()
         torch.cuda.cudart().cudaProfilerStop()
+    if args.dump_outputs and rank == 0:   # before anything else reuses the output buffers of the timed steps
+        dump_outputs(args.dump_outputs, ("ids", "scores", "parts", "counts") if use_lib else ("ids", "scores", "parts") if multi else ("ids", "scores", "counts"), last)
     ms_total = step_ev[0].elapsed_time(step_ev[-1])
     per_step = None if pipelined else [step_ev[i].elapsed_time(step_ev[i + 1]) for i in range(args.steps)]
     launches = L.nidx_launch_count() - launches0
@@ -796,4 +810,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True   # the benchmark writes nothing into the source tree, which may be read-only
     sys.exit(main())

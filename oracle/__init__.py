@@ -12,9 +12,12 @@ third-party crate absent from /root/reference and no reference test asserts a BM
 """
 from __future__ import annotations
 
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -24,22 +27,34 @@ SIM_DOT, SIM_COSINE, SIM_L2 = 0, 1, 2
 BM25_OR, BM25_AND = 0, 1
 
 _lib = None
+_native_path = None
 
 
 def build(native: bool = False) -> str:
-    """Compile the oracle (gcc only).  Returns the path of the shared object."""
-    target = "native" if native else "liboracle.so"
-    subprocess.run(["make", "-s", "-C", _HERE, target], check=True)
-    return os.path.join(_HERE, "liboracle_native.so" if native else "liboracle.so")
+    """Compile the oracle (gcc only).  Returns the path of the shared object.  The -march=native build is only valid on the
+    machine that compiles it, so it goes to a temporary directory of this process (removed at exit), never into the source tree,
+    which may be read-only; it is compiled once per process and must load here."""
+    global _native_path
+    if not native:
+        subprocess.run(["make", "-s", "-C", _HERE, "liboracle.so"], check=True)
+        return os.path.join(_HERE, "liboracle.so")
+    if _native_path is None:
+        tmp = tempfile.mkdtemp(prefix="oracle_native_")
+        atexit.register(shutil.rmtree, tmp, True)
+        path = os.path.join(tmp, "liboracle_native.so")
+        subprocess.run(["make", "-s", "-C", _HERE, "native", f"NATIVE_OUT={path}"], check=True)
+        C.CDLL(path)
+        _native_path = path
+    return _native_path
 
 
 def lib(native: bool = False):
     global _lib
     if _lib is not None and not native:
         return _lib
-    path = os.path.join(_HERE, "liboracle_native.so" if native else "liboracle.so")
+    path = build(True) if native else os.path.join(_HERE, "liboracle.so")
     if not os.path.exists(path):
-        build(native)
+        build()
     L = C.CDLL(path)
     L.oracle_dot.restype = C.c_float
     L.oracle_dot_f64.restype = C.c_double

@@ -1,40 +1,34 @@
-"""The constants the hot path takes from the reference, read from the reference's own Rust sources (build container only; skipped
-elsewhere) and compared with what the mirror, the oracle and the CUDA sources use."""
+"""The constants the hot path takes from the reference, as read from the reference's own Rust sources into
+tests/golden/reference_facts.json (tests/golden/make_reference_facts.py), compared with what the mirror, the oracle and the CUDA
+sources use."""
+import json
 import os
 import re
 
-import pytest
-
-REF = "/root/reference/nidx/nidx_vector/src"
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
-
-
-def rust_const(path, name):
-    m = re.search(rf"const\s+{name}\s*:\s*\w+\s*=\s*([0-9.]+)\s*;", open(os.path.join(REF, path)).read())
-    assert m, (path, name)
-    return float(m.group(1))
+REF = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_facts.json")))["nidx_vector"]
 
 
 def test_hnsw_parameters():
     """hnsw/params.rs:34-46: M, M_MAX, M_MAX_0, EF_CONSTRUCTION, EF_SEARCH and prune_m = m * 95 / 100 = the mirror's and the library's defaults."""
     from nucliadb_b200 import vector as V
 
+    p = REF["hnsw_params"]
     cfg = V.VectorConfig(dimension=8)
-    assert cfg.m == rust_const("hnsw/params.rs", "M") == rust_const("hnsw/params.rs", "M_MAX")
-    assert cfg.m0 == rust_const("hnsw/params.rs", "M_MAX_0")
-    assert cfg.ef_construction == rust_const("hnsw/params.rs", "EF_CONSTRUCTION")
-    assert cfg.ef_search == rust_const("hnsw/params.rs", "EF_SEARCH")
-    assert re.search(r"fn prune_m\(m: usize\) -> usize \{\s*m \* 95 / 100", open(os.path.join(REF, "hnsw/params.rs")).read())
-    assert "mmax * 95 / 100" in open(os.path.join(ROOT, "nucliadb_b200", "csrc", "hnsw_build.cuh")).read()
+    assert cfg.m == p["M"] == p["M_MAX"]
+    assert cfg.m0 == p["M_MAX_0"]
+    assert cfg.ef_construction == p["EF_CONSTRUCTION"]
+    assert cfg.ef_search == p["EF_SEARCH"]
+    num, den = p["prune_m_ratio"]
+    assert f"mmax * {num} / {den}" in open(os.path.join(ROOT, "nucliadb_b200", "csrc", "hnsw_build.cuh")).read()
     header = open(os.path.join(ROOT, "include", "nidx_b200.h")).read()
-    for field, want in (("m;", 30), ("m0;", 60), ("ef_construction;", 100), ("ef_search;", 30)):
+    for field, want in (("m;", p["M"]), ("m0;", p["M_MAX_0"]), ("ef_construction;", p["EF_CONSTRUCTION"]), ("ef_search;", p["EF_SEARCH"])):
         assert re.search(rf"int32_t {re.escape(field)}[^\n]*0 => {want} \*/", header), field
 
 
 def test_rabitq_constants():
     """vector_types/rabitq.rs:30-36: EPSILON, RERANKING_FACTOR, RERANKING_LIMIT in the kernels, the host code and the oracle."""
-    eps, fac, lim = rust_const("vector_types/rabitq.rs", "EPSILON"), rust_const("vector_types/rabitq.rs", "RERANKING_FACTOR"), rust_const("vector_types/rabitq.rs", "RERANKING_LIMIT")
+    eps, fac, lim = REF["rabitq"]["EPSILON"], REF["rabitq"]["RERANKING_FACTOR"], REF["rabitq"]["RERANKING_LIMIT"]
     cu = open(os.path.join(ROOT, "nucliadb_b200", "csrc", "rabitq.cuh")).read()
     assert float(re.search(r"RABITQ_EPSILON = ([0-9.]+)f", cu).group(1)) == eps
     assert float(re.search(r"RABITQ_EPSILON = ([0-9.]+)f", open(os.path.join(ROOT, "oracle", "rabitq.hpp")).read()).group(1)) == eps
@@ -45,27 +39,25 @@ def test_rabitq_constants():
 
 
 def test_cost_model_matches_the_reference_source():
-    """segment.rs:626-660 use_hnsw: the constants of the reference's function body (16, * 3 / 4, / 2, ln - 2.0) appear in api.cu's
-    use_hnsw_cost, and the function agrees with a literal Python transcription of the Rust on a grid."""
-    import math
+    """segment.rs:626-660 use_hnsw: the constants of the reference's function body (16, * 3 / 4, / 2, ln - 2.0) as stored, and the
+    oracle's restatement agrees with a literal Python transcription of the Rust, built from those constants, on a grid."""
+    import numpy as np
 
     import oracle as O
 
-    seg = open(os.path.join(REF, "segment.rs")).read()
-    body = seg[seg.index("fn use_hnsw("):]
-    body = body[: body.index("\n}\n")]
-    assert "full_cost = 16;" in body and "RERANKING_FACTOR * 3 / 4" in body and "RERANKING_FACTOR / 2" in body and ".ln() - 2.0).powi(2)" in body
+    c = REF["use_hnsw"]
+    rq, plain = c["with_rabitq"], c["without_rabitq"]
+    assert (rq["full_cost"], rq["search_mult_of_reranking_factor"], rq["rerank_divisor_of_reranking_factor"]) == (16, [3, 4], 2)
+    assert (plain["full_cost"], plain["search_mult"], plain["rerank_mult"]) == (1, 1, 0) and (c["log_offset"], c["log_power"]) == (2.0, 2)
+    fac = REF["rabitq"]["RERANKING_FACTOR"]
 
-    def f32(x):
-        import numpy as np
-
-        return np.float32(x)
-
-    def ref(total, matching, k, rq, M=30):
-        full, smul, rmul = (16, 100 * 3 // 4, 100 // 2) if rq else (1, 1, 0)
-        import numpy as np
-
-        hnsw_rq = (np.log(f32(total)) - f32(2.0)) ** 2 * np.log(f32(k)) * f32(smul)
+    def ref(total, matching, k, has_rq, M=30):
+        if has_rq:
+            num, den = rq["search_mult_of_reranking_factor"]
+            full, smul, rmul = rq["full_cost"], fac * num // den, fac // rq["rerank_divisor_of_reranking_factor"]
+        else:
+            full, smul, rmul = plain["full_cost"], plain["search_mult"], plain["rerank_mult"]
+        hnsw_rq = (np.log(np.float32(total)) - np.float32(c["log_offset"])) ** c["log_power"] * np.log(np.float32(k)) * np.float32(smul)
         hnsw_full = k * rmul + k * M * total // matching
         hnsw_cost = (int(hnsw_rq) if hnsw_rq > 0 else 0) + hnsw_full * full
         return hnsw_cost < matching + k * rmul * full
@@ -74,19 +66,17 @@ def test_cost_model_matches_the_reference_source():
         for frac in (1.0, 0.3, 0.01, 0.0001):
             matching = max(1, int(total * frac))
             for k in (1, 10, 100):
-                for rq in (False, True):
-                    assert bool(O.use_hnsw(total, matching, k, has_rabitq=rq, M=30)) == bool(ref(total, matching, k, rq)), (total, matching, k, rq)
-    assert math.isfinite(1.0)
+                for has_rq in (False, True):
+                    assert bool(O.use_hnsw(total, matching, k, has_rabitq=has_rq, M=30)) == bool(ref(total, matching, k, has_rq)), (total, matching, k, has_rq)
 
 
 def test_segment_file_names():
     """The v2 segment directory's file names (hnsw/disk/v2.rs:64-65, data_store/v2/*.rs): what the library and the mirror read and write."""
-    want = {"hnsw.graph": ("hnsw/disk/v2.rs", "GRAPH_FILENAME"), "hnsw.edges": ("hnsw/disk/v2.rs", "EDGES_FILENAME"),
-            "vectors.bin": ("data_store/v2/vector_store.rs", "FILENAME"), "vectors.quant": ("data_store/v2/quant_vector_store.rs", "FILENAME"),
-            "paragraphs.bin": ("data_store/v2/paragraph_store.rs", "FILENAME_DATA"), "paragraphs.pos": ("data_store/v2/paragraph_store.rs", "FILENAME_POS")}
+    want = {"hnsw.graph": "hnsw/disk/v2.rs:GRAPH_FILENAME", "hnsw.edges": "hnsw/disk/v2.rs:EDGES_FILENAME",
+            "vectors.bin": "data_store/v2/vector_store.rs:FILENAME", "vectors.quant": "data_store/v2/quant_vector_store.rs:FILENAME",
+            "paragraphs.bin": "data_store/v2/paragraph_store.rs:FILENAME_DATA", "paragraphs.pos": "data_store/v2/paragraph_store.rs:FILENAME_POS"}
     ours = open(os.path.join(ROOT, "nucliadb_b200", "csrc", "segment_io.hpp")).read() + open(os.path.join(ROOT, "nucliadb_b200", "csrc", "api.cu")).read() + \
         open(os.path.join(ROOT, "nucliadb_b200", "paragraph_store.py")).read() + open(os.path.join(ROOT, "nucliadb_b200", "vector.py")).read()
-    for name, (path, const) in want.items():
-        m = re.search(rf'const\s+{const}\s*:\s*&str\s*=\s*"([^"]+)"', open(os.path.join(REF, path)).read())
-        assert m and m.group(1) == name, (path, const)
+    for name, const in want.items():
+        assert REF["segment_file_names"][const] == name, const
         assert f'"/{name}"' in ours or f'"{name}"' in ours, name

@@ -216,26 +216,18 @@ def test_paragraph_store_round_trip_property():
 
 
 def test_nidx_binding_has_the_reference_surface():
-    """nidx/nidx_binding/nidx_binding.pyi:15-71 read here (the build container has the reference; elsewhere the test is skipped):
-    every method of the reference's NidxBinding exists with the same parameter names, and both port attributes are declared."""
-    import ast
+    """nidx/nidx_binding/nidx_binding.pyi:15-71, as read into tests/golden/reference_facts.json: every method of the reference's
+    NidxBinding exists with the same parameter names, and both port attributes are declared."""
     import inspect
+    import json
 
-    import pytest
-
-    pyi = "/root/reference/nidx/nidx_binding/nidx_binding.pyi"
-    if not os.path.exists(pyi):
-        pytest.skip("reference tree not present")
     import nidx_binding
 
-    cls = next(n for n in ast.parse(open(pyi).read()).body if isinstance(n, ast.ClassDef) and n.name == "NidxBinding")
-    for node in cls.body:
-        if isinstance(node, ast.FunctionDef):
-            ours = getattr(nidx_binding.NidxBinding, node.name)
-            want = [a.arg for a in node.args.args]
-            got = list(inspect.signature(ours).parameters)
-            assert got == want, (node.name, got, want)
-        elif isinstance(node, ast.AnnAssign):
-            assert node.target.id in ("searcher_port", "api_port")
+    ref = json.load(open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_facts.json")))["nidx_binding"]["NidxBinding"]
+    assert ref["methods"]
+    for name, want in ref["methods"].items():
+        got = list(inspect.signature(getattr(nidx_binding.NidxBinding, name)).parameters)
+        assert got == want, (name, got, want)
+    assert sorted(ref["attributes"]) == ["api_port", "searcher_port"]
     src = inspect.getsource(nidx_binding.NidxBinding.__init__)
     assert "self.searcher_port" in src and "self.api_port" in src

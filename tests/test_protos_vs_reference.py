@@ -1,94 +1,23 @@
 """The hand-built protobuf descriptors (nucliadb_b200/nidx_protos.py: there is no protoc here) against the reference's own .proto files
-(nidx/nidx_protos/*.proto), parsed with a small reader: every field declared by hand must exist in the reference message with the same
-number, type and cardinality -- the wire compatibility of the outer boundary (NidxSearcher.Search / NidxApi.NewShard / IndexMessage).
-Reads /root/reference: runs in the build container, skipped where the reference tree is absent."""
+(nidx/nidx_protos/*.proto), as parsed into tests/golden/reference_facts.json by tests/golden/make_reference_facts.py: every field
+declared by hand must exist in the reference message with the same number, type and cardinality -- the wire compatibility of the
+outer boundary (NidxSearcher.Search / NidxApi.NewShard / IndexMessage)."""
+import json
 import os
-import re
 
-import pytest
 from google.protobuf import descriptor_pb2
 
-REF = "/root/reference/nidx/nidx_protos"
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REF = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_facts.json")))["nidx_protos"]
 _F = descriptor_pb2.FieldDescriptorProto
 _SCALAR = {_F.TYPE_STRING: "string", _F.TYPE_BYTES: "bytes", _F.TYPE_INT32: "int32", _F.TYPE_INT64: "int64", _F.TYPE_UINT32: "uint32",
            _F.TYPE_UINT64: "uint64", _F.TYPE_FLOAT: "float", _F.TYPE_BOOL: "bool", _F.TYPE_DOUBLE: "double"}
 
 
-def parse_proto(path):
-    """-> ({full message name: {field: (number, type, repeated)}}, {full enum name: {value name: number}}); handles nesting, oneof, map<>."""
-    text = re.sub(r"//[^\n]*", "", open(path).read())
-    text = re.sub(r"/\*.*?\*/", "", text, flags=re.S)
-    pkg = re.search(r"\bpackage\s+([\w.]+)\s*;", text).group(1)
-    tokens = re.findall(r"[{};=<>,]|[\w.]+|\"[^\"]*\"|\[[^\]]*\]", text)
-    msgs, enums = {}, {}
-    stack = []          # [(kind, name)]
-    i = 0
-    while i < len(tokens):
-        t = tokens[i]
-        if t in ("message", "enum", "oneof", "service") and tokens[i + 2] == "{":
-            name = tokens[i + 1]
-            if t == "oneof":
-                stack.append(("oneof", None))
-            else:
-                scope = ".".join([pkg] + [n for k, n in stack if k == "message"] + [name])
-                stack.append((t, name))
-                if t == "message":
-                    msgs[scope] = {}
-                elif t == "enum":
-                    enums[scope] = {}
-            i += 3
-            continue
-        if t == ";":
-            i += 1
-            continue
-        if t == "{":                 # any other block (rpc bodies, option blocks)
-            stack.append(("block", None))
-            i += 1
-            continue
-        if t == "}":
-            stack.pop()
-            i += 1
-            continue
-        kinds = [k for k, _ in stack]
-        if kinds and kinds[-1] == "enum" and i + 2 < len(tokens) and tokens[i + 1] == "=":
-            scope = ".".join([pkg] + [n for k, n in stack if k in ("message", "enum")])
-            enums[scope][t] = int(tokens[i + 2])
-            i += 3
-            continue
-        if kinds and kinds[-1] in ("message", "oneof") and t not in ("option", "reserved", "extensions"):
-            scope = ".".join([pkg] + [n for k, n in stack if k == "message"])
-            rep = False
-            j = i
-            if tokens[j] in ("repeated", "optional"):
-                rep = tokens[j] == "repeated"
-                j += 1
-            if tokens[j] == "map" and tokens[j + 1] == "<":
-                ktype, vtype, name, num = tokens[j + 2], tokens[j + 4], tokens[j + 6], int(tokens[j + 8])
-                msgs[scope][name] = (num, f"map<{ktype},{vtype}>", True)
-                i = j + 9
-            elif j + 3 < len(tokens) and tokens[j + 2] == "=":
-                msgs[scope][tokens[j + 1]] = (int(tokens[j + 3]), tokens[j], rep)
-                i = j + 4
-            else:
-                i += 1
-                continue
-            while i < len(tokens) and tokens[i] != ";" and tokens[i] not in ("}", "{"):
-                i += 1
-            continue
-        i += 1
-    return msgs, enums
-
-
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present")
 def test_hand_built_descriptors_match_the_reference_protos():
     from nucliadb_b200 import nidx_protos as P
 
-    ref_msgs, ref_enums = {}, {}
-    for f in os.listdir(REF):
-        if f.endswith(".proto"):
-            m, e = parse_proto(os.path.join(REF, f))
-            ref_msgs.update(m)
-            ref_enums.update(e)
+    ref_msgs, ref_enums = REF["messages"], REF["enums"]
     checked = 0
 
     def short(type_name, scope):
@@ -140,7 +69,6 @@ def test_hand_built_descriptors_match_the_reference_protos():
                 assert ref_enums[full].get(v.name) == v.number, (full, v.name)
     assert seen_files == 4 and checked > 80
     # the two rpc paths
-    nidx = open(os.path.join(REF, "nidx.proto")).read()
-    assert re.search(r"service\s+NidxSearcher\s*{[^}]*rpc\s+Search\s*\(\s*nodereader\.SearchRequest\s*\)\s*returns\s*\(\s*nodereader\.SearchResponse\s*\)", nidx)
-    assert re.search(r"rpc\s+NewShard\s*\(\s*nodewriter\.NewShardRequest\s*\)\s*returns\s*\(\s*noderesources\.ShardCreated\s*\)", nidx)
+    assert REF["services"]["nidx.NidxSearcher"]["Search"] == ["nodereader.SearchRequest", "nodereader.SearchResponse"]
+    assert REF["services"]["nidx.NidxApi"]["NewShard"] == ["nodewriter.NewShardRequest", "noderesources.ShardCreated"]
     assert P.SEARCH_METHOD == "/nidx.NidxSearcher/Search" and P.NEW_SHARD_METHOD == "/nidx.NidxApi/NewShard"
